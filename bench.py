@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's outputs as DIR/<name>.npy
     (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 Workload ("ns", the configuration the metric is quoted on): a batch of 8 meshes of 69,938 faces each
@@ -292,7 +293,7 @@ def run_ours(args, rank, local_rank, world):
 
     def step():
         f = fwd()
-        return _C.rasterize_meshes_backward(fv, f[0], gz, gb, gd, False, False)
+        return f, _C.rasterize_meshes_backward(fv, f[0], gz, gb, gd, False, False)
 
     def barrier():
         if world > 1:
@@ -308,9 +309,13 @@ def run_ours(args, rank, local_rank, world):
     with ClockSampler(local_rank) as clocks:
         e0.record()
         for _ in range(args.steps):
-            step()
+            last = None  # the previous step's outputs are released before the step allocates its own
+            last = step()
         e1.record()
         barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
+    last = None
     launches = lib.b200r_kernel_launch_count() - launches0
     ms = e0.elapsed_time(e1)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
@@ -586,6 +591,34 @@ def run_ours(args, rank, local_rank, world):
             "impl": "pytorch3d_b200",
         }
         print(json.dumps(line), flush=True)
+
+
+DUMP_BYTES = 60 * 1000 * 1000  # what --dump-outputs may write: with the .npy headers, under 64 MB in all
+
+
+def _seeded_rows(n, keep, seed=0):
+    """`keep` of `n` row indices, a fixed seeded sample in ascending order (all of them when keep >= n)."""
+    if keep >= n:
+        return torch.arange(n)
+    return torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+
+
+def dump_outputs(out_dir, frags, grad_face_verts):
+    """Writes what the timed step returns -- the Fragments (pix_to_face, zbuf, bary_coords, dists) and the gradient
+    w.r.t. face_verts -- as out_dir/<name>.npy in float32 (pix_to_face in float64: exact).  Each half of DUMP_BYTES
+    holds one of the two; where an output does not fit, a fixed seeded sample of its pixels (all K slots) or faces is
+    written, the same rows for every build, so that two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    p2f = frags[0]
+    N, H, W, K = (int(v) for v in p2f.shape)
+    pix = _seeded_rows(N * H * W, DUMP_BYTES // 2 // (K * (8 + 4 + 12 + 4))).to(p2f.device)
+    for name, t in zip(("pix_to_face", "zbuf", "bary_coords", "dists"), frags):
+        rows = t.reshape((N * H * W,) + tuple(t.shape[3:]))[pix]
+        np.save(os.path.join(out_dir, name + ".npy"),
+                rows.to(torch.float64 if name == "pix_to_face" else torch.float32).cpu().numpy())
+    F = int(grad_face_verts.shape[0])
+    faces = _seeded_rows(F, DUMP_BYTES // 2 // 36).to(grad_face_verts.device)
+    np.save(os.path.join(out_dir, "grad_face_verts.npy"), grad_face_verts[faces].float().cpu().numpy())
 
 
 def _time_ms(fn, steps=20, warm=3):
@@ -940,6 +973,7 @@ def main():
     ap.add_argument("--skip-host-abi", action="store_true")
     ap.add_argument("--skip-others", action="store_true", help="skip the other configs / reference-CUDA legs")
     ap.add_argument("--skip-c4", action="store_true", help="skip the sharded config-4 leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 

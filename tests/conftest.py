@@ -26,12 +26,12 @@ def pytest_collection_modifyitems(config, items):
 @pytest.fixture(scope="session")
 def golden():
     import numpy as np
-    path = os.path.join(ROOT, "tests", "golden", "raster_golden.npz")
-    data = np.load(path)
     cases = {}
-    for key in data.files:
-        case, field = key.rsplit("/", 1)
-        cases.setdefault(case, {})[field] = data[key]
+    for name in ("raster_golden.npz", "clip_golden.npz"):  # (two files: each stays under 1 MB)
+        data = np.load(os.path.join(ROOT, "tests", "golden", name))
+        for key in data.files:
+            case, field = key.rsplit("/", 1)
+            cases.setdefault(case, {})[field] = data[key]
     return cases
 
 

@@ -1,10 +1,11 @@
 """Compositing of point features (SURVEY.md 8f-2: alpha, weighted sum, normalised weighted sum): oracle pinned to the
-reference CPU ops; CUDA path against oracle / reference."""
+reference CPU ops; CUDA path against oracle / reference (stored outputs, tests/golden/make_reference_outputs.py)."""
 import numpy as np
 import pytest
 import torch
 
 import oracle
+from helpers import case_key, digest, reference_outputs
 
 
 def scene(N, K, H, W, C, P, seed, frac_empty=0.3):
@@ -19,24 +20,26 @@ def scene(N, K, H, W, C, P, seed, frac_empty=0.3):
     return feats, alphas, idx
 
 
+REF_CASES = [(2, 5, 9, 11, 3, 40), (1, 1, 4, 4, 1, 5), (1, 10, 16, 8, 4, 100)]  # N, K, H, W, C, P
+CUDA_CASES = [(2, 5, 9, 11, 3, 40, False), (2, 10, 33, 17, 4, 500, True), (1, 1, 4, 4, 1, 5, False),
+              (3, 8, 20, 20, 8, 300, True)]  # N, K, H, W, C, P, permuted
+
+
 @pytest.fixture(scope="module")
 def ref_cpu():
-    m = oracle.load_reference(cuda=False)
-    if m is None or not hasattr(m, "accum_alphacomposite"):
-        pytest.skip("reference CPU build without compositing not present")
-    return m
+    """Digests of the reference's C++ CPU ops on these seeded scenes (tests/golden/make_reference_outputs.py cpu)."""
+    return reference_outputs("reference_cpu")
 
 
-@pytest.mark.parametrize("N,K,H,W,C,P", [(2, 5, 9, 11, 3, 40), (1, 1, 4, 4, 1, 5), (1, 10, 16, 8, 4, 100)])
+@pytest.mark.parametrize("N,K,H,W,C,P", REF_CASES)
 def test_oracle_equals_reference_cpu(ref_cpu, N, K, H, W, C, P):
+    want = ref_cpu[case_key("alpha", N, K, H, W, C, P)]
     feats, alphas, idx = scene(N, K, H, W, C, P, seed=K)
-    want = ref_cpu.accum_alphacomposite(feats, alphas, idx)
     got = oracle.alpha_composite(feats.numpy(), alphas.numpy(), idx.numpy(), arith=oracle.ARITH_CPU)
-    assert np.array_equal(got, want.numpy())
-    go = torch.rand(want.shape, generator=torch.Generator().manual_seed(1))
-    rf, ra = ref_cpu.accum_alphacomposite_backward(go, feats, alphas, idx)
+    assert digest(got) == str(want["forward"])
+    go = torch.rand(got.shape, generator=torch.Generator().manual_seed(1))
     of, oa = oracle.alpha_composite_backward(go.numpy(), feats.numpy(), alphas.numpy(), idx.numpy())
-    assert np.array_equal(of, rf.numpy()) and np.array_equal(oa, ra.numpy())
+    assert digest(of, oa) == str(want["backward"])
 
 
 def test_oracle_closed_form():
@@ -51,8 +54,7 @@ def test_oracle_closed_form():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("N,K,H,W,C,P,permuted", [(2, 5, 9, 11, 3, 40, False), (2, 10, 33, 17, 4, 500, True),
-                                                  (1, 1, 4, 4, 1, 5, False), (3, 8, 20, 20, 8, 300, True)])
+@pytest.mark.parametrize("N,K,H,W,C,P,permuted", CUDA_CASES)
 def test_cuda_forward_backward(built_lib, N, K, H, W, C, P, permuted):
     from pytorch3d_b200 import _C, compositing
     dev = torch.device("cuda:0")
@@ -67,10 +69,8 @@ def test_cuda_forward_backward(built_lib, N, K, H, W, C, P, permuted):
     out = _C.accum_alphacomposite(fd, ad, idd)
     want = oracle.alpha_composite(feats.numpy(), alphas.numpy(), idx.numpy(), arith=oracle.ARITH_CUDA)
     assert np.array_equal(out.cpu().numpy(), want), "forward must be bit-identical to the CUDA-form oracle"
-    ref = oracle.load_reference(cuda=True)
-    if ref is not None and hasattr(ref, "accum_alphacomposite"):
-        r = ref.accum_alphacomposite(fd, alphas.to(dev), idx.to(dev))
-        assert torch.equal(out, r), "forward must be bit-identical to the reference CUDA kernel"
+    ref = reference_outputs("reference_cuda")[case_key("alpha_cuda", N, K, H, W, C, P)]
+    assert digest(out) == str(ref["forward"]), "forward must be bit-identical to the reference CUDA kernel"
     go = torch.rand(out.shape, generator=torch.Generator().manual_seed(1))
     gf, ga = _C.accum_alphacomposite_backward(go.to(dev), fd, ad, idd)
     of, oa = oracle.alpha_composite_backward(go.numpy(), feats.numpy(), alphas.numpy(), idx.numpy())
@@ -111,28 +111,22 @@ def test_points_renderer_pipeline(built_lib):
 # ------------------------------------------------------------------------------------ weighted sums
 
 @pytest.mark.parametrize("norm", [False, True])
-@pytest.mark.parametrize("N,K,H,W,C,P", [(2, 5, 9, 11, 3, 40), (1, 1, 4, 4, 1, 5), (1, 10, 16, 8, 4, 100)])
+@pytest.mark.parametrize("N,K,H,W,C,P", REF_CASES)
 def test_weighted_sum_oracle_equals_reference_cpu(ref_cpu, norm, N, K, H, W, C, P):
-    if not hasattr(ref_cpu, "accum_weightedsum"):
-        pytest.skip("reference CPU build without the weighted-sum ops")
+    want = ref_cpu[case_key("weighted_sum", norm, N, K, H, W, C, P)]
     feats, alphas, idx = scene(N, K, H, W, C, P, seed=K + 7)
     if norm:
         alphas[:, :, 0, 0] = 1e-6  # total below the 1e-4 floor
-    fwd = ref_cpu.accum_weightedsumnorm if norm else ref_cpu.accum_weightedsum
-    bwd = ref_cpu.accum_weightedsumnorm_backward if norm else ref_cpu.accum_weightedsum_backward
-    want = fwd(feats, alphas, idx)
     got = oracle.weighted_sum(feats.numpy(), alphas.numpy(), idx.numpy(), norm=norm)
-    assert np.array_equal(got, want.numpy())
-    go = torch.rand(want.shape, generator=torch.Generator().manual_seed(1))
-    rf, ra = bwd(go, feats, alphas, idx)
+    assert digest(got) == str(want["forward"])
+    go = torch.rand(got.shape, generator=torch.Generator().manual_seed(1))
     of, oa = oracle.weighted_sum_backward(go.numpy(), feats.numpy(), alphas.numpy(), idx.numpy(), norm=norm)
-    assert np.array_equal(of, rf.numpy()) and np.array_equal(oa, ra.numpy())
+    assert digest(of, oa) == str(want["backward"])
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("norm", [False, True])
-@pytest.mark.parametrize("N,K,H,W,C,P,permuted", [(2, 5, 9, 11, 3, 40, False), (2, 10, 33, 17, 4, 500, True),
-                                                  (1, 1, 4, 4, 1, 5, False), (3, 8, 20, 20, 8, 300, True)])
+@pytest.mark.parametrize("N,K,H,W,C,P,permuted", CUDA_CASES)
 def test_weighted_sum_cuda_forward_backward(built_lib, norm, N, K, H, W, C, P, permuted):
     from pytorch3d_b200 import _C, compositing
     dev = torch.device("cuda:0")
@@ -150,10 +144,8 @@ def test_weighted_sum_cuda_forward_backward(built_lib, norm, N, K, H, W, C, P, p
     out = fwd(fd, ad, idd)
     want = oracle.weighted_sum(feats.numpy(), alphas.numpy(), idx.numpy(), norm=norm)
     assert np.array_equal(out.cpu().numpy(), want), "forward must be bit-identical to the oracle"
-    ref = oracle.load_reference(cuda=True)
-    if ref is not None and hasattr(ref, "accum_weightedsum"):
-        rfwd = ref.accum_weightedsumnorm if norm else ref.accum_weightedsum
-        assert torch.equal(out, rfwd(fd, alphas.to(dev), idx.to(dev))), "forward must equal the reference CUDA kernel"
+    ref = reference_outputs("reference_cuda")[case_key("weighted_sum_cuda", norm, N, K, H, W, C, P)]
+    assert digest(out) == str(ref["forward"]), "forward must equal the reference CUDA kernel"
     go = torch.rand(out.shape, generator=torch.Generator().manual_seed(1))
     gf, ga = bwd(go.to(dev), fd, ad, idd)
     of, oa = oracle.weighted_sum_backward(go.numpy(), feats.numpy(), alphas.numpy(), idx.numpy(), norm=norm)

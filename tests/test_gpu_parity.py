@@ -1,5 +1,5 @@
-"""Parity of the CUDA path (called through the C ABI) with the oracle, the golden fixtures and -- when
-oracle/_ref/ref_raster_cuda.so travelled to the box -- the reference's own CUDA kernels.
+"""Parity of the CUDA path (called through the C ABI) with the oracle, the golden fixtures and the reference's own CUDA
+kernels (their outputs on these seeded inputs, stored by tests/golden/make_reference_outputs.py).
 
 Bar: pix_to_face / idx bit-exact; zbuf / bary / dists bit-exact too against the CUDA-flavoured oracle
 (identical arithmetic), <= 1e-5 against fixtures produced by the reference's CPU build; gradients within
@@ -9,7 +9,7 @@ import pytest
 import torch
 
 import oracle
-from helpers import assert_frag_equal, rand_faces, rand_points, split, upstream
+from helpers import assert_frag_equal, case_key, digest, rand_faces, rand_points, reference_outputs, split, upstream
 
 pytestmark = pytest.mark.gpu
 
@@ -30,7 +30,7 @@ def ops(built_lib):
 
 @pytest.fixture(scope="module")
 def ref_cuda():
-    return oracle.load_reference(cuda=True)  # None on a box without the prebuilt reference
+    return reference_outputs("reference_cuda")
 
 
 def run_mesh(ops, dev, fv, first, num, size, blur, K, persp=0, clip=0, cull=0, nb=None):
@@ -99,11 +99,7 @@ def test_mesh_forward_structured_with_z_ties(ops, dev, ref_cuda):
     lex = oracle.rasterize_meshes(fv.numpy(), first.numpy(), num.numpy(), (256, 256), 1e-4, 8,
                                   arith=oracle.ARITH_CUDA, select=oracle.SELECT_CPU)
     assert (lex[0] != o[0]).sum() > 0, "scene is expected to contain ties (guards the test's purpose)"
-    if ref_cuda is not None:
-        nb = torch.full((fv.shape[0],), -1, dtype=torch.int64, device=dev)
-        r = ref_cuda.rasterize_meshes(fv.to(dev), first.to(dev), num.to(dev), nb, (256, 256), 1e-4, 8, 0, 0, False,
-                                      False, False)
-        assert_frag_equal(mine, r, "torus vs reference CUDA (naive)")
+    assert digest(*mine) == str(ref_cuda["torus_ties"]["forward"]), "torus vs reference CUDA (naive)"
 
 
 def test_config1_ico_sphere(ops, dev):
@@ -140,14 +136,10 @@ def test_mesh_golden_fixtures(ops, dev, golden):
 
 @pytest.mark.parametrize("persp,clip,cull,blur,K,H,W,F,N", MESH_MATRIX[:6])
 def test_mesh_forward_equals_reference_cuda(ops, dev, ref_cuda, persp, clip, cull, blur, K, H, W, F, N):
-    if ref_cuda is None:
-        pytest.skip("reference CUDA build not present")
     fv, first, num = rand_faces(F, N, seed=K + H)
     mine = run_mesh(ops, dev, fv, first, num, (H, W), blur, K, persp, clip, cull)
-    nb = torch.full((F,), -1, dtype=torch.int64, device=dev)
-    r = ref_cuda.rasterize_meshes(fv.to(dev), first.to(dev), num.to(dev), nb, (H, W), blur, K, 0, 0, bool(persp),
-                                  bool(clip), bool(cull))
-    assert_frag_equal(mine, r, "mine vs reference CUDA naive")
+    want = ref_cuda[case_key("mesh_forward", persp, clip, cull, blur, K, H, W, F, N)]["forward"]
+    assert digest(*mine) == str(want), "mine vs reference CUDA naive"
 
 
 def test_mesh_edge_cases(ops, dev):
@@ -226,7 +218,10 @@ def test_more_images_than_grid_z(ops, dev):
     assert np.abs(pgrad - pref).max() <= 1e-4 * max(np.abs(pref).max(), 1e-6)
 
 
-@pytest.mark.parametrize("persp,clip,blur", [(0, 0, 1e-3), (1, 0, 1e-3), (0, 1, 1e-3), (1, 1, 0.0), (1, 1, 1e-3)])
+BACKWARD_CASES = [(0, 0, 1e-3), (1, 0, 1e-3), (0, 1, 1e-3), (1, 1, 0.0), (1, 1, 1e-3)]  # persp, clip, blur
+
+
+@pytest.mark.parametrize("persp,clip,blur", BACKWARD_CASES)
 def test_mesh_backward(ops, dev, ref_cuda, persp, clip, blur):
     from pytorch3d_b200 import synthetic
     m = synthetic.torus_batch(2, 24, 24, seed=3)
@@ -248,22 +243,19 @@ def test_mesh_backward(ops, dev, ref_cuda, persp, clip, blur):
         assert ok.mean() >= 0.98
         # second witness: the reference's own C++ CPU backward (rasterize_meshes_cpu.cpp:391-532), which applies the clip
         # backward to the corrected barycentrics like this build (its CUDA kernel does not: DESIGN.md 5)
-        ref_cpu = oracle.load_reference(cuda=False)
-        if ref_cpu is not None:
-            rc = ref_cpu.rasterize_meshes_backward(fv, frag[0].cpu(), gz, gb, gd, True, True).numpy()
-            err_c = np.abs(mine - rc).reshape(nf, -1).max(1)
-            mag_c = np.abs(rc).reshape(nf, -1).max(1)
-            ok_c = err_c <= 2e-3 * np.maximum(mag_c, 1e-3 * np.median(mag_c))
-            assert ok_c.mean() >= 0.98
+        rc = ref_cuda[case_key("mesh_backward", persp, clip, blur)]["grad_face_verts"]
+        err_c = np.abs(mine - rc).reshape(nf, -1).max(1)
+        mag_c = np.abs(rc).reshape(nf, -1).max(1)
+        ok_c = err_c <= 2e-3 * np.maximum(mag_c, 1e-3 * np.median(mag_c))
+        assert ok_c.mean() >= 0.98
         return
     scale = mag.max()
     assert err.max() <= 2e-3 * scale
     np.testing.assert_allclose(mine, want, rtol=2e-3, atol=2e-4 * scale)
-    if ref_cuda is not None and not (persp and clip):
+    if not (persp and clip):
         # (with both flags the reference CUDA kernel feeds the uncorrected barycentrics to the clip
         # backward, rasterize_meshes.cu:527-529; we follow the forward-consistent CPU form)
-        r = ref_cuda.rasterize_meshes_backward(fv.to(dev), frag[0], gz.to(dev), gb.to(dev), gd.to(dev), bool(persp),
-                                               bool(clip)).cpu().numpy()
+        r = ref_cuda[case_key("mesh_backward", persp, clip, blur)]["grad_face_verts"]
         np.testing.assert_allclose(mine, r, rtol=2e-3, atol=2e-4 * scale)
 
 
@@ -346,9 +338,8 @@ def test_points_forward_equals_oracle(ops, dev, ref_cuda, P, N, H, W, K):
     mine = ops.rasterize_points(pts.to(dev), first.to(dev), num.to(dev), (H, W), rad.to(dev), K, 0, 0)
     o = oracle.rasterize_points(pts.numpy(), first.numpy(), num.numpy(), (H, W), rad.numpy(), K, **CUDA)
     assert_frag_equal(mine, o, "points vs oracle")
-    if ref_cuda is not None:
-        r = ref_cuda.rasterize_points(pts.to(dev), first.to(dev), num.to(dev), (H, W), rad.to(dev), K, 0, 0)
-        assert_frag_equal(mine, r, "points vs reference CUDA naive")
+    want = ref_cuda[case_key("points_forward", P, N, H, W, K)]["forward"]
+    assert digest(*mine) == str(want), "points vs reference CUDA naive"
 
 
 def test_points_golden_fixtures(ops, dev, golden):
@@ -400,7 +391,7 @@ def test_points_autograd_wrapper(ops, dev):
 
 def test_full_size_properties(ops, dev, ref_cuda):
     """North-star size (8 x 69,938 faces, 512^2, K=8): size-independent properties, plus exact equality
-    with the reference CUDA op when it is available on the box."""
+    with the reference CUDA op."""
     from pytorch3d_b200 import synthetic
     m = synthetic.torus_batch(8, 187, 187, seed=0)
     fv = synthetic.face_verts_of(m).to(dev)
@@ -433,10 +424,7 @@ def test_full_size_properties(ops, dev, ref_cuda):
     # z is the barycentric interpolation of the face's vertex depths
     zi = (bary * fv[p2f.clamp_min(0)][..., 2]).sum(-1)
     assert (zi - zbuf)[valid].abs().max() < 1e-5
-    if ref_cuda is not None:
-        nb = torch.full((fv.shape[0],), -1, dtype=torch.int64, device=dev)
-        r = ref_cuda.rasterize_meshes(fv, first, num, nb, (512, 512), 0.0, 8, 32, 14000, False, False, False)
-        assert_frag_equal(a, r, "north-star vs reference CUDA (coarse-to-fine)")
+    assert digest(*a) == str(ref_cuda["full_size"]["forward"]), "north-star vs reference CUDA (coarse-to-fine)"
     # backward: linear in the upstream gradients
     gz, gb, gd = (t.to(dev) for t in upstream([zbuf.shape, bary.shape, dists.shape]))
     g1 = ops.rasterize_meshes_backward(fv, p2f, gz, gb, gd, False, False)

@@ -1,10 +1,22 @@
 """interpolate_face_attributes (SURVEY.md 8f-3): oracle vs fixtures from the reference's CPU path; CUDA path vs oracle
-and, when present, vs the reference's CUDA op."""
+and vs the reference's CUDA op (stored outputs, tests/golden/make_reference_outputs.py)."""
 import numpy as np
 import pytest
 import torch
 
 import oracle
+from helpers import case_key, digest, reference_outputs
+
+CUDA_CASES = [(2, 9, 11, 3, 50, 3), (1, 4, 4, 1, 6, 1), (2, 16, 16, 4, 300, 16)]  # N, H, W, K, F, D
+
+
+def scene(N, H, W, K, F, D):
+    """(pix_to_face, bary, attrs) and the generator that made them (it seeds the upstream gradient next)."""
+    g = torch.Generator().manual_seed(F + D)
+    p2f = torch.randint(-1, F, (N, H, W, K), generator=g)
+    bary = torch.rand(N, H, W, K, 3, generator=g)
+    attrs = torch.randn(F, 3, D, generator=g)
+    return p2f, bary, attrs, g
 
 
 def test_oracle_matches_reference_fixtures(golden):
@@ -30,22 +42,17 @@ def test_invalid_shapes_raise(built_lib):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("N,H,W,K,F,D", [(2, 9, 11, 3, 50, 3), (1, 4, 4, 1, 6, 1), (2, 16, 16, 4, 300, 16)])
+@pytest.mark.parametrize("N,H,W,K,F,D", CUDA_CASES)
 def test_cuda_forward_backward(built_lib, N, H, W, K, F, D):
     from pytorch3d_b200 import _C
     from pytorch3d_b200.interp_face_attrs import interpolate_face_attributes
     dev = torch.device("cuda:0")
-    g = torch.Generator().manual_seed(F + D)
-    p2f = torch.randint(-1, F, (N, H, W, K), generator=g)
-    bary = torch.rand(N, H, W, K, 3, generator=g)
-    attrs = torch.randn(F, 3, D, generator=g)
+    p2f, bary, attrs, g = scene(N, H, W, K, F, D)
     out = _C.interp_face_attrs_forward(p2f.reshape(-1).to(dev), bary.reshape(-1, 3).to(dev), attrs.to(dev))
     want = oracle.interp_face_attrs(p2f.numpy(), bary.numpy(), attrs.numpy(), arith=oracle.ARITH_CUDA)
     assert np.array_equal(out.cpu().numpy(), want), "forward must be bit-identical to the CUDA-form oracle"
-    ref = oracle.load_reference(cuda=True)
-    if ref is not None and hasattr(ref, "interp_face_attrs_forward"):
-        r = ref.interp_face_attrs_forward(p2f.reshape(-1).to(dev), bary.reshape(-1, 3).to(dev), attrs.to(dev))
-        assert torch.equal(out, r), "forward must be bit-identical to the reference CUDA kernel"
+    ref = reference_outputs("reference_cuda")[case_key("interp", N, H, W, K, F, D)]
+    assert digest(out) == str(ref["forward"]), "forward must be bit-identical to the reference CUDA kernel"
     go = torch.randn(out.shape, generator=g)
     gb, ga = _C.interp_face_attrs_backward(p2f.reshape(-1).to(dev), bary.reshape(-1, 3).to(dev), attrs.to(dev),
                                            go.to(dev))

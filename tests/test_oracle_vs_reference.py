@@ -1,12 +1,12 @@
 """Pins the C oracle (oracle/raster_oracle.c): against the committed golden fixtures produced by running
-the reference (tests/golden/make_golden.py), and -- when the reference sources are present so that
-oracle/_ref/ref_raster_cpu.so exists -- bit-for-bit against the reference's own C++ CPU ops."""
+the reference (tests/golden/make_golden.py), and bit-for-bit against the reference's own C++ CPU ops (their outputs'
+digests, stored by tests/golden/make_reference_outputs.py)."""
 import numpy as np
 import pytest
 import torch
 
 import oracle
-from helpers import rand_faces, rand_points, upstream
+from helpers import case_key, digest, rand_faces, rand_points, reference_outputs, upstream
 
 MESH_CPP = lambda g: sorted(k for k in g if k.startswith("mesh/") and "/cpp" in k)  # noqa: E731
 MESH_PY = lambda g: sorted(k for k in g if k.startswith("mesh/") and "/python" in k)  # noqa: E731
@@ -81,54 +81,53 @@ def test_golden_points(golden):
             assert np.array_equal(g, c["grad_points"]), name
 
 
+REF_MESH_CASES = [  # persp, clip, cull, blur, K, H, W
+    (0, 0, 0, 0.0, 4, 32, 32), (1, 0, 0, 1e-3, 8, 33, 47), (0, 1, 1, 1e-2, 3, 64, 40), (1, 1, 0, 1e-4, 8, 48, 48),
+    (1, 1, 1, 0.05, 150, 16, 16)]
+REF_POINT_CASES = [(1, 16, 16), (5, 32, 48), (10, 40, 24)]  # K, H, W
+
+
+def neighbor_table():
+    nb = torch.full((300,), -1, dtype=torch.int64)
+    nb[0:100:2] = torch.arange(1, 100, 2)
+    nb[1:100:2] = torch.arange(0, 100, 2)
+    return nb
+
+
 @pytest.fixture(scope="module")
 def ref_cpu():
-    m = oracle.load_reference(cuda=False)
-    if m is None:
-        pytest.skip("oracle/_ref/ref_raster_cpu.so not built (reference sources absent on this machine)")
-    return m
+    """Digests of the reference's C++ CPU ops on these seeded scenes (tests/golden/make_reference_outputs.py cpu)."""
+    return reference_outputs("reference_cpu")
 
 
-@pytest.mark.parametrize("persp,clip,cull,blur,K,H,W", [
-    (0, 0, 0, 0.0, 4, 32, 32), (1, 0, 0, 1e-3, 8, 33, 47), (0, 1, 1, 1e-2, 3, 64, 40), (1, 1, 0, 1e-4, 8, 48, 48),
-    (1, 1, 1, 0.05, 150, 16, 16)])
+@pytest.mark.parametrize("persp,clip,cull,blur,K,H,W", REF_MESH_CASES)
 def test_oracle_equals_reference_cpu_meshes(ref_cpu, persp, clip, cull, blur, K, H, W):
+    want = ref_cpu[case_key("meshes", persp, clip, cull, blur, K, H, W)]
     fv, first, num = rand_faces(400, 2, seed=K + H)
-    nb = torch.full((fv.shape[0],), -1, dtype=torch.int64)
-    r = ref_cpu.rasterize_meshes(fv, first, num, nb, (H, W), blur, K, 0, 0, bool(persp), bool(clip), bool(cull))
     o = oracle.rasterize_meshes(fv.numpy(), first.numpy(), num.numpy(), (H, W), blur, K, persp, clip, cull)
-    for a, b in zip(r, o):
-        assert np.array_equal(a.numpy(), b)
-    gz, gb, gd = upstream([r[1].shape, r[2].shape, r[3].shape])
-    rg = ref_cpu.rasterize_meshes_backward(fv, r[0], gz, gb, gd, bool(persp), bool(clip))
+    assert digest(*o) == str(want["forward"])
+    gz, gb, gd = upstream([o[1].shape, o[2].shape, o[3].shape])
     og = oracle.rasterize_meshes_backward(fv.numpy(), o[0], gz.numpy(), gb.numpy(), gd.numpy(), persp, clip)
-    assert np.array_equal(rg.numpy(), og)
+    assert digest(og) == str(want["backward"])
 
 
 def test_oracle_equals_reference_cpu_neighbors(ref_cpu):
     """clipped_faces_neighbor_idx semantics (rasterize_meshes_cpu.cpp:249-277)."""
     fv, first, num = rand_faces(300, 1, seed=7, scale=0.35)
-    nb = torch.full((300,), -1, dtype=torch.int64)
-    nb[0:100:2] = torch.arange(1, 100, 2)
-    nb[1:100:2] = torch.arange(0, 100, 2)
-    r = ref_cpu.rasterize_meshes(fv, first, num, nb, (32, 32), 1e-2, 4, 0, 0, False, False, False)
     o = oracle.rasterize_meshes(fv.numpy(), first.numpy(), num.numpy(), (32, 32), 1e-2, 4,
-                                clipped_faces_neighbor_idx=nb.numpy())
-    for a, b in zip(r, o):
-        assert np.array_equal(a.numpy(), b)
+                                clipped_faces_neighbor_idx=neighbor_table().numpy())
+    assert digest(*o) == str(ref_cpu["neighbors"]["forward"])
 
 
-@pytest.mark.parametrize("K,H,W", [(1, 16, 16), (5, 32, 48), (10, 40, 24)])
+@pytest.mark.parametrize("K,H,W", REF_POINT_CASES)
 def test_oracle_equals_reference_cpu_points(ref_cpu, K, H, W):
+    want = ref_cpu[case_key("points", K, H, W)]
     pts, first, num, rad = rand_points(1500, 2, seed=K)
-    r = ref_cpu.rasterize_points(pts, first, num, (H, W), rad, K, 0, 0)
     o = oracle.rasterize_points(pts.numpy(), first.numpy(), num.numpy(), (H, W), rad.numpy(), K)
-    for a, b in zip(r, o):
-        assert np.array_equal(a.numpy(), b)
-    gz, gd = upstream([r[1].shape, r[2].shape])
-    rg = ref_cpu.rasterize_points_backward(pts, r[0], gz, gd)
+    assert digest(*o) == str(want["forward"])
+    gz, gd = upstream([o[1].shape, o[2].shape])
     og = oracle.rasterize_points_backward(pts.numpy(), o[0], gz.numpy(), gd.numpy())
-    assert np.array_equal(rg.numpy(), og)
+    assert digest(og) == str(want["backward"])
 
 
 def test_oracle_flavours_agree_without_ties():
