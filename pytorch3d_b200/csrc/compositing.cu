@@ -9,7 +9,8 @@
 // Redesign: the reference runs one thread per (pixel, channel), recomputes the transmittance chain per channel,
 // accumulates with atomics into a pre-zeroed result, and its backward issues O(K^2) atomics per (pixel, channel)
 // on grad_alphas.  Here one thread owns a pixel: the chain is walked once, every output is written exactly once
-// (no zero-fill, no atomics on result / grad_alphas), grad_alphas uses a suffix sum (O(K) per pixel), and only
+// (no zero-fill, no atomics on result / grad_alphas), grad_alphas uses a suffix sum (O(K) per pixel, with the forward's
+// front-to-back transmittance parked between its two passes), and only
 // grad_features -- a genuine scatter -- uses atomics.  The forward value is bit-identical to the reference kernel:
 // same products ((f * cum) * alpha), same ascending-k summation order.
 // `alphas` / `points_idx` are addressed through element strides, because the renderer passes permuted views of the
@@ -24,6 +25,15 @@ struct Strides4 {
 };
 
 constexpr float kCompEps = 1e-9f;  // alpha_composite.cu:20
+
+// The compositing backward walks a pixel's slots twice: front to back for the transmittances, back to front for the
+// gradients.  Between the two passes each thread parks its pixel's transmittances in a column of shared memory when
+// K <= kParkMaxK (at most 32 KB per CTA of 256; the read-back is then an on-chip load, which the `memory` clobber of
+// the reductions would otherwise turn into one L2 round trip per slot), else in the slot's own gradient output.
+constexpr int kParkMaxK = 32;
+extern __shared__ float park_smem[];
+
+static size_t park_smem_bytes(int K) { return K <= kParkMaxK ? (size_t)K * 256 * sizeof(float) : 0; }
 
 // One 16-byte reduction for the four channels of a point (point-major features, C = 4): sm_90+ vector atomics.
 __device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
@@ -98,12 +108,20 @@ __global__ void __launch_bounds__(256)
     float* ga = grad_alphas + (int64_t)n * K * plane + (int64_t)y * W + x;     // + k * plane (contiguous N,K,H,W)
     const bool pm4 = C == 4 && fs_c == 1 && fs_p == 4 &&
                      ((reinterpret_cast<uintptr_t>(features) | reinterpret_cast<uintptr_t>(grad_features)) & 15u) == 0;
-    // transmittance before the last valid slot, then walk the slots backwards keeping the suffix sum
+    // first pass: the transmittance in front of each valid slot, cum_k = prod_{l<k, valid} (1 - alpha_l), built front
+    // to back exactly as the forward builds it and parked (see kParkMaxK; grad_alphas[k] belongs to this thread);
+    // then walk the slots backwards keeping the suffix sum
     //   S_k = sum_{t>k} cum_t * alpha_t * A_t,   A_t = sum_c grad_out_c * feat[c, idx_t]
     // grad_alpha_k = cum_k * A_k - S_k / (1 - alpha_k + eps)          (alpha_composite.cu:112-134, summed over c)
+    // (recovering cum_k by dividing the full product by (1 - alpha_k) loses every slot once that product underflows:
+    // K = 150 at alpha 0.5, or a dozen near-opaque hits)
+    float* park = K <= kParkMaxK ? park_smem + threadIdx.x : ga;
+    const int64_t ps = K <= kParkMaxK ? (int64_t)blockDim.x : plane;
     float cum = 1.0f;
     for (int k = 0; k < K; ++k) {
-      if (ip[k * si.k] >= 0) cum *= 1.0f - ap[k * sa.k];
+      if (ip[k * si.k] < 0) continue;
+      park[k * ps] = cum;
+      cum = fmul(cum, fsub(1.0f, ap[k * sa.k]));
     }
     float suffix = 0.0f;
     for (int k = K - 1; k >= 0; --k) {
@@ -114,16 +132,7 @@ __global__ void __launch_bounds__(256)
       }
       const float a = ap[k * sa.k];
       const float one_minus = 1.0f - a;
-      // cum currently includes slot k: undo it (exactly what the forward chain had before slot k, up to rounding;
-      // recomputed from scratch when the factor is ~0 to avoid dividing by it)
-      float cum_k;
-      if (fabsf(one_minus) > 1e-6f) {
-        cum_k = cum / one_minus;
-      } else {
-        cum_k = 1.0f;
-        for (int l = 0; l < k; ++l)
-          if (ip[l * si.k] >= 0) cum_k *= 1.0f - ap[l * sa.k];
-      }
+      const float cum_k = park[k * ps];
       float A = 0.0f;
       const float w = cum_k * a;
       if (pm4) {  // point-major features, four channels: one 16-byte load and one 16-byte reduction per hit
@@ -140,7 +149,6 @@ __global__ void __launch_bounds__(256)
       }
       ga[k * plane] = cum_k * A - suffix / (one_minus + kCompEps);
       suffix += w * A;
-      cum = cum_k;
     }
   }
 }
@@ -335,10 +343,16 @@ __global__ void __launch_bounds__(256)
 #pragma unroll
       for (int c = 0; c < CMAX; ++c) g[c] = c < C ? go[c * plane] : 0.0f;
     }
-    // (the arithmetic of alpha_composite_backward_kernel above, with alpha_k = 1 - d_k * inv)
+    // (the arithmetic of alpha_composite_backward_kernel above, with alpha_k = 1 - d_k * inv; cum_k parked in shared
+    // memory or in grad_dists[k] between the two passes)
+    float* park = K <= kParkMaxK ? park_smem + threadIdx.x : gd;
+    const int ps = K <= kParkMaxK ? (int)blockDim.x : 1;
     float cum = 1.0f;
-    for (int k = 0; k < K; ++k)
-      if (ip[k] >= 0) cum *= 1.0f - fsub(1.0f, fmul(dp[k], inv));
+    for (int k = 0; k < K; ++k) {
+      if (ip[k] < 0) continue;
+      park[k * ps] = cum;
+      cum = fmul(cum, fsub(1.0f, fsub(1.0f, fmul(dp[k], inv))));
+    }
     float suffix = 0.0f;
     for (int k = K - 1; k >= 0; --k) {
       const int id = ip[k];
@@ -348,14 +362,7 @@ __global__ void __launch_bounds__(256)
       }
       const float a = fsub(1.0f, fmul(dp[k], inv));
       const float one_minus = 1.0f - a;
-      float cum_k;
-      if (fabsf(one_minus) > 1e-6f) {
-        cum_k = cum / one_minus;
-      } else {
-        cum_k = 1.0f;
-        for (int l = 0; l < k; ++l)
-          if (ip[l] >= 0) cum_k *= 1.0f - fsub(1.0f, fmul(dp[l], inv));
-      }
+      const float cum_k = park[k * ps];
       float A = 0.0f;
       const float w = cum_k * a;
       if (CMAX > 0) {
@@ -386,7 +393,6 @@ __global__ void __launch_bounds__(256)
       const float ga = cum_k * A - suffix / (one_minus + kCompEps);
       gd[k] = fmul(-ga, inv);  // d(1 - d * inv) / dd = -inv
       suffix += w * A;
-      cum = cum_k;
     }
   }
 }
@@ -432,7 +438,7 @@ extern "C" int b200r_points_alpha_render_backward(const float* grad_images, cons
   int64_t blocks = (total + 255) / 256;
   if (blocks > 148 * 32) blocks = 148 * 32;
 #define B200R_PAR_BWD(CM)                                                                                       \
-  points_alpha_render_backward_kernel<CM><<<(unsigned)blocks, 256, 0, stream>>>(                                \
+  points_alpha_render_backward_kernel<CM><<<(unsigned)blocks, 256, park_smem_bytes(K), stream>>>(                                \
       grad_images, features, C, feature_stride_c, feature_stride_p, idx, dists, radius2, N, K, H, W,            \
       grad_features, grad_dists)
   if (C <= 4)
@@ -512,7 +518,7 @@ extern "C" int b200r_alpha_composite_backward_strided(const float* grad_out, con
   const Strides4 si = {idx_strides[0], idx_strides[1], idx_strides[2], idx_strides[3]};
   int64_t blocks = (total + 255) / 256;
   if (blocks > 148 * 32) blocks = 148 * 32;
-  alpha_composite_backward_kernel<<<(unsigned)blocks, 256, 0, stream>>>(grad_out, features, C, feature_stride_c,
+  alpha_composite_backward_kernel<<<(unsigned)blocks, 256, park_smem_bytes(K), stream>>>(grad_out, features, C, feature_stride_c,
                                                                       feature_stride_p, alphas, sa, points_idx, si, N, K,
                                                                       H, W, grad_features, grad_alphas);
   B200R_LAUNCHED("alpha_composite_backward_kernel");
