@@ -53,7 +53,6 @@ __device__ __forceinline__ bool rect_empty(uint2 r) { return (r.x & 0xFFFFu) > (
 
 // The tile counters are zeroed by a kernel the setup pass is chained to (programmatic dependent launch) instead of a memset
 // node: the setup pass's loads and arithmetic overlap it and wait only before their first atomic (binning -1.8 us).
-#ifndef B200R_EXP_MEMSET_NODE
 static __global__ void __launch_bounds__(256) zero_ints_kernel(int* __restrict__ p, int64_t n) {
   const int64_t i = ((int64_t)blockIdx.x * 256 + threadIdx.x) * 4;
   pdl_trigger();
@@ -62,7 +61,6 @@ static __global__ void __launch_bounds__(256) zero_ints_kernel(int* __restrict__
   else
     for (int64_t j = i; j < n && j < i + 4; ++j) p[j] = 0;
 }
-#endif
 
 // Count one element per tile of its rectangle.  Called by ALL 32 lanes of a warp (lanes without work pass an
 // empty rectangle): consecutive elements of a packed mesh are neighbours on screen, so most lanes of a warp
@@ -90,7 +88,6 @@ __device__ __forceinline__ void warp_count_rect(uint2 r, int n, int TY, int TX, 
   for (int i = 0; i < rounds; ++i) {
     const bool act = i < ntile;
     const int t = act ? (n * TY + ty) * TX + tx : -1 - lane;  // inactive lanes get unique keys
-#ifndef B200R_EXP_AGG_MATCH
     // runs of consecutive lanes with the same tile -- a shuffle and two votes -- instead of __match_any_sync, whose result
     // the atomic waited for (17 % of the setup kernel's stall samples; north-star binning 44.7 -> 40.8 us, config 2 23.6 ->
     // 21.5 us); equal tiles that are not adjacent in the warp cost one more atomic
@@ -101,10 +98,6 @@ __device__ __forceinline__ void warp_count_rect(uint2 r, int n, int TY, int TX, 
       const unsigned after = lane == 31 ? 0u : conts >> (lane + 1);
       atomicAdd(tile_count + t, 1 + (__ffs((int)~after) - 1));
     }
-#else
-    const unsigned grp = __match_any_sync(0xffffffffu, t);
-    if (act && lane == __ffs(grp) - 1) atomicAdd(tile_count + t, __popc(grp));
-#endif
     if (++tx > tx1) {
       tx = tx0;
       ++ty;
@@ -122,15 +115,8 @@ __device__ __forceinline__ void warp_count_rect(uint2 r, int n, int TY, int TX, 
 // keeps neighbouring tiles -- which share most of their faces' records -- in flight together (an arbitrary order inside
 // the classes cost config 5 11 %).  Three classes: longer than the mean non-empty list, shorter, empty; the per-class
 // ranks of all tiles come from ONE block scan of a packed counter (3 x 21 bits).
-#ifdef B200R_EXP_ORDER4  // (experiment: four classes -- > 2 x mean, > mean, shorter, empty -- of 16-bit counters)
-constexpr int ORDER_BITS = 16, ORDER_CLASSES = 4;
-__device__ __forceinline__ int order_class(int count, int mean) {
-  return count <= 0 ? 3 : (count > 2 * mean ? 0 : (count > mean ? 1 : 2));
-}
-#else
 constexpr int ORDER_BITS = 21, ORDER_CLASSES = 3;
 __device__ __forceinline__ int order_class(int count, int mean) { return count <= 0 ? 2 : (count > mean ? 0 : 1); }
-#endif
 __device__ __forceinline__ unsigned long long order_key(int count, int mean) {
   return 1ull << (ORDER_BITS * order_class(count, mean));
 }
@@ -330,7 +316,6 @@ static __global__ void __launch_bounds__(256)
   for (int i = 0; i < rounds; ++i) {
     const bool act = i < ntile;
     const int t = act ? (n * TY + ty) * TX + tx : -1 - lane;
-#ifndef B200R_EXP_AGG_MATCH
     const int tprev = __shfl_up_sync(0xffffffffu, t, 1);
     const bool cont = act && lane > 0 && t == tprev;
     const unsigned conts = __ballot_sync(0xffffffffu, cont);
@@ -345,15 +330,6 @@ static __global__ void __launch_bounds__(256)
     base = __shfl_sync(0xffffffffu, base, leader);
     if (act) {
       const int pos = base + (lane - leader);
-#else
-    const unsigned grp = __match_any_sync(0xffffffffu, t);
-    const int leader = __ffs(grp) - 1;
-    int base = 0;
-    if (act && lane == leader) base = atomicAdd(cursor + t, __popc(grp));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (act) {
-      const int pos = base + __popc(grp & ((1u << lane) - 1u));
-#endif
       if (pos >= 0 && (int64_t)pos < capacity) pairs[pos] = (int)e;  // (pos < 0: saturated / wrapped cursor)
     }
     if (++tx > tx1) {
@@ -370,10 +346,7 @@ static __global__ void __launch_bounds__(256)
 // chunk's first one (a chunk may straddle clouds) use the global counters directly.
 // (elements per CTA: config 3 -- 8 x 100 k points -- binning 42.0 us with 2048 = 391 CTAs, 36.7 / 37.4 us with 1024, 37.9 us
 // with 512, 48.1 us with 256: more CTAs than SMs x resident CTAs against more global atomics per element)
-#ifndef B200R_BIN_CHUNK
-#define B200R_BIN_CHUNK 1024
-#endif
-constexpr int BIN_CHUNK = B200R_BIN_CHUNK;  // elements per CTA (4 per thread)
+constexpr int BIN_CHUNK = 1024;        // elements per CTA (4 per thread)
 constexpr int BIN_MAX_TILES = 8192;      // tiles per image that the private histogram can hold (32 KB)
 
 // Fill: local histogram -> one returning global atomic per touched tile reserves the CTA's range in the tile's
@@ -407,12 +380,6 @@ static __global__ void __launch_bounds__(256)
       for (int tx = tx0; tx <= tx1; ++tx) atomicAdd(hist + ty * TX + tx, 1);
   }
   __syncthreads();
-#ifdef B200R_EXP_PFILL_SERIAL
-  for (int t = tid; t < T; t += 256) {
-    const int c = hist[t];
-    if (c > 0) hist[t] = atomicAdd(cursor + n0 * T + t, c);  // start of this CTA's range in the tile's segment
-  }
-#else
   // (four returning atomics in flight per thread: each would wait for its own round trip to L2 otherwise)
   for (int t0 = tid; t0 < T; t0 += 4 * 256) {
     int c[4], b[4];
@@ -424,7 +391,6 @@ static __global__ void __launch_bounds__(256)
     for (int u = 0; u < 4; ++u)
       if (c[u] > 0) hist[t0 + u * 256] = b[u];  // start of this CTA's range in the tile's segment
   }
-#endif
   __syncthreads();
 #pragma unroll
   for (int i = 0; i < BIN_CHUNK / 256; ++i) {
@@ -561,43 +527,6 @@ __device__ __forceinline__ void cta_sort_segment(int* seg, int n, int* s_keys, i
   }
   if (in_smem)
     for (int i = threadIdx.x; i < n; i += NT) seg[i] = s_keys[i];
-  __syncthreads();
-}
-
-// A tile list of any length put in ascending order of 64-bit keys built by `make_key(element)`; the keys live in shared
-// memory (`keys`, room for n of them), the list itself is rewritten in that order.  Used by the mesh fine pass to walk a
-// tile's faces front to back (key = (nearest vertex depth, face)).
-template <int NT, class MakeKey>
-__device__ __forceinline__ void cta_sort_segment_by_key(int* seg, int n, unsigned long long* keys, MakeKey make_key) {
-  for (int i = threadIdx.x; i < n; i += NT) keys[i] = make_key(seg[i]);
-  __syncthreads();
-  for (int k = 2; (k >> 1) < n; k <<= 1) {
-    for (int i = threadIdx.x; i < n; i += NT) {  // mirror step
-      const int j = i ^ (k - 1);
-      if (j > i && j < n) {
-        const unsigned long long a = keys[i], b = keys[j];
-        if (b < a) {
-          keys[i] = b;
-          keys[j] = a;
-        }
-      }
-    }
-    __syncthreads();
-    for (int d = k >> 2; d > 0; d >>= 1) {
-      for (int i = threadIdx.x; i < n; i += NT) {
-        const int j = i ^ d;
-        if (j > i && j < n) {
-          const unsigned long long a = keys[i], b = keys[j];
-          if (b < a) {
-            keys[i] = b;
-            keys[j] = a;
-          }
-        }
-      }
-      __syncthreads();
-    }
-  }
-  for (int i = threadIdx.x; i < n; i += NT) seg[i] = (int)(unsigned)(keys[i] & 0xffffffffull);
   __syncthreads();
 }
 

@@ -24,10 +24,9 @@ namespace b200r {
 constexpr int SETUP_FACES = 256;  // faces per CTA in the setup pass (one per thread)
 // Tile of the mesh FORWARD pass (binning + fine kernels): FTW x FTH pixels, one thread per pixel, warps own 8x4
 // footprints.  (The backward kernels and the point rasterizer keep TILE x TILE = 16 x 16.)
-#ifndef B200R_MESH_TILE_H
-#define B200R_MESH_TILE_H 16
-#endif
-constexpr int FTW = 16, FTH = B200R_MESH_TILE_H, FTHREADS = FTW * FTH;
+// (16 x 8 tiles were measured: north-star fine 141.3 -> 141.9 us, binning 45 -> 51 us, config 5 9.3 -> 10.3 ms; only
+// config 2 gains, 139.7 -> 123.4 us.)
+constexpr int FTW = 16, FTH = 16, FTHREADS = FTW * FTH;
 static_assert(FTH == 16 || FTH == 8, "16x16 or 16x8 tiles");
 constexpr int CHUNK = FTHREADS;   // faces staged per round in the fine pass (one per thread)
 constexpr int SMEMQ_MAX_K = 32;   // largest K served by the shared-memory queue kernel (mesh_fine_smemq_kernel)
@@ -97,11 +96,10 @@ __device__ __forceinline__ void exact_pixel_range(float vmin, float vmax, int S,
 // INDEXED (the fused entry point): the faces are given as (verts, faces); the kernel gathers the three vertices
 // of each face itself -- what `verts_packed[faces_packed]` does in the reference's wrapper
 // (rasterize_meshes.py:144-148) -- and also writes the gathered (F,3,3) array for the backward pass.
-#ifndef B200R_SETUP_CTAS
-#define B200R_SETUP_CTAS 1
-#endif
+// Resident CTAs per SM the register budget is set for (6 / 8: binning 44.8 -> 45.6 / 46.8 us).
+constexpr int SETUP_CTAS = 1;
 template <bool INDEXED>
-__global__ void __launch_bounds__(SETUP_FACES, B200R_SETUP_CTAS)
+__global__ void __launch_bounds__(SETUP_FACES, SETUP_CTAS)
     mesh_setup_count_kernel(const float* __restrict__ face_verts, const float* __restrict__ verts, int64_t V,
                             const int64_t* __restrict__ faces, float* __restrict__ face_verts_out,
                             const int64_t* __restrict__ neighbor, int64_t F, const int64_t* __restrict__ first,
@@ -166,9 +164,7 @@ __global__ void __launch_bounds__(SETUP_FACES, B200R_SETUP_CTAS)
                               : make_float4(__int_as_float(rng.x), __int_as_float(rng.y), __int_as_float(rng.z),
                                             __int_as_float(rng.w));
   }
-#ifndef B200R_EXP_MEMSET_NODE
   pdl_wait();  // the counters are zeroed by the kernel this one is chained to (see zero_ints_kernel)
-#endif
   warp_count_rect(r, n, TY, TX, tile_count, tid & 31);  // all lanes participate
 }
 
@@ -200,14 +196,10 @@ __device__ __forceinline__ bool eval_pixel_face(float px, float py, const Face& 
   if (clip) bary_clip(c0, c1, c2);
   const float pz = ffma(f.z2, c2, ffma(f.z0, c0, fmul(f.z1, c1)));
   if (!(pz >= 0.0f)) return false;  // behind the image plane (:163)
-#ifdef B200R_EXP_NOEARLYZ
-  (void)full; (void)max_z;
-#else
   if (full && !(pz < max_z)) {
     if (WATCH && pz == max_z) flag_tie();
     return false;
   }
-#endif
   const bool inside = w0 > 0.0f && w1 > 0.0f && w2 > 0.0f;
   if (!inside && !(blur_radius > 0.0f)) return false;  // dist >= 0 >= blur_radius always rejects (:175)
   const float dist = point_tri_dist(px, py, f);
@@ -536,20 +528,15 @@ struct FineStage {
     float4 box[CHUNK];                          // blur > 0: blur-expanded boxes (pass A)
     unsigned mask[CHUNK / 32][FTHREADS];        // blur = 0: per pixel (thread), one bit per staged face
     int sort_buf[2 * FTHREADS];                 // exchange buffers of cta_sort256 (before the chunk is staged)
-    unsigned long long sort_buf64[2 * FTHREADS];  // ... of cta_sort256_u64
   } u;
   unsigned rng[CHUNK];                          // blur = 0: tile-local pixel rectangle c_lo | c_hi<<8 | r_lo<<16 | r_hi<<24
   float col[FTW], row[FTH];                     // NDC coordinates of the tile's pixel columns / rows
   int tie;                                      // see flag_tie()
-  unsigned char tie_lane[FTHREADS];             // ... and which pixels (threads) raised it
 };
 
 __device__ __forceinline__ void flag_tie() {
-#ifndef B200R_EXP_NOWATCH  // (timing experiment of tools/variant_time.py: no tie watching at all)
   extern __shared__ __align__(16) unsigned char smem_raw[];
   reinterpret_cast<FineStage*>(smem_raw)->tie = 1;
-  reinterpret_cast<FineStage*>(smem_raw)->tie_lane[threadIdx.x] = 1;
-#endif
 }
 
 // Full-sector output stores.  A pixel's K values of one buffer are P 16-byte pieces; the pixels of two adjacent
@@ -720,36 +707,23 @@ __device__ __forceinline__ float face_depth_lower_bound(const float4 fa, const f
 // triangles of a quad extrapolate to the same depth) and with clipped-face neighbours (whose replace-in-queue rule
 // depends on the order by itself) the list is sorted up front.  Either way the result is the one the sorted walk
 // gives; sorting every list cost 30 % of the kernel's instructions.
-// `order`: ORDER_ARRIVAL (the list as the fill pass left it), ORDER_INDEX (ascending face index: the reference's order)
-// or ORDER_DEPTH (ascending nearest-vertex depth: front to back).  `active`: this thread's pixel takes part in the walk
-// (its queue is updated); inactive threads still help to stage.  `scratch_ints`: how much of the kernel's shared memory,
-// from its start, a long-list sort may use (everything on the first walk of a tile; only the staging area when queue
-// payload of an earlier walk must survive).
-enum { ORDER_ARRIVAL = 0, ORDER_INDEX = 1, ORDER_DEPTH = 2 };
+// `order`: ORDER_ARRIVAL (the list as the fill pass left it) or ORDER_INDEX (ascending face index: the reference's
+// order).  `valid`: this thread's pixel lies in the image (its queue is updated); the others still help to stage.
+enum { ORDER_ARRIVAL = 0, ORDER_INDEX = 1 };
 
 template <class Q, bool NB, bool SCAN>
 __device__ __forceinline__ void fine_tile_body(const FineParams& p, FineStage& sh, Q& q, int tile_x, int tile_y, int n,
-                                               int seg_begin, int count, bool overflow, int order, bool active,
-                                               int scratch_ints, int lc, int lr) {
+                                               int seg_begin, int count, bool overflow, int order, bool valid, int lc,
+                                               int lr) {
   const int tid = threadIdx.x, lane = tid & 31;
   const bool persp = p.persp != 0, clip = p.clip != 0;
   const float blur_radius = p.blur_radius;
-  const bool valid = active;
   // (an overflowed tile walks the mesh's own faces: already in order)
   const bool sorted_walk = order == ORDER_INDEX;
   const bool sort_staged = sorted_walk && !overflow && count <= CHUNK;
-  const bool depth_staged = order == ORDER_DEPTH && count <= CHUNK;
-  const float4* rec = p.rec;
-  // nearest vertex depth of a listed face (listed faces are drawable: z > 0, the float's bits are ordered), then its index
-  auto depth_key = [rec](int f) {
-    const float4 c = __ldg(rec + (int64_t)f * 4 + 2);
-    return ((unsigned long long)__float_as_uint(fminf(fminf(c.x, c.y), c.z)) << 32) | (unsigned)f;
-  };
-  // (the long-list sorts use the kernel's shared memory as scratch: nothing lives in that part yet / any more)
+  // (the long-list sort uses the kernel's shared memory as scratch: nothing lives there yet / any more)
   if (sorted_walk && !overflow && count > CHUNK)
-    cta_sort_segment<FTHREADS>(p.pairs + seg_begin, count, reinterpret_cast<int*>(&sh), scratch_ints);
-  if (order == ORDER_DEPTH && count > CHUNK)
-    cta_sort_segment_by_key<FTHREADS>(p.pairs + seg_begin, count, reinterpret_cast<unsigned long long*>(&sh), depth_key);
+    cta_sort_segment<FTHREADS>(p.pairs + seg_begin, count, reinterpret_cast<int*>(&sh), p.smem_ints);
   // NDC coordinates of the tile's 16 pixel columns and rows (two IEEE divisions each): computed once per tile
   // by 32 threads, read by every thread after the barriers of the first chunk
   if (tid < FTW + FTH) {
@@ -758,10 +732,7 @@ __device__ __forceinline__ void fine_tile_body(const FineParams& p, FineStage& s
     else
       sh.row[tid - FTW] = pix_to_ndc(p.H - 1 - (tile_y * FTH + tid - FTW), p.H, p.ry);
   }
-  if (!sorted_walk) {
-    if (tid == FTW + FTH) sh.tie = 0;
-    sh.tie_lane[tid] = 0;
-  }
+  if (!sorted_walk && tid == FTW + FTH) sh.tie = 0;
 
   for (int base = 0; base < count; base += CHUNK) {
     const int nc = min(CHUNK, count - base);
@@ -772,12 +743,6 @@ __device__ __forceinline__ void fine_tile_body(const FineParams& p, FineStage& s
     if (sort_staged) {
       f = cta_sort256<FTHREADS>(f, nc, sh.u.sort_buf);
       if (nc > 32) __syncthreads();  // the exchange buffers alias the masks / boxes written next
-    } else if (depth_staged) {
-      unsigned long long key = ~0ull;
-      if (tid < nc) key = depth_key(f);
-      key = cta_sort256_u64<FTHREADS>(key, nc, sh.u.sort_buf64);
-      if (nc > 32) __syncthreads();
-      f = (int)(unsigned)(key & 0xffffffffull);
     }
     if (tid < nc) {
       const float4* r = p.rec + (int64_t)f * 4;
@@ -810,10 +775,7 @@ __device__ __forceinline__ void fine_tile_body(const FineParams& p, FineStage& s
       //      leaves the candidates of every pixel in ascending face order.  (Measured on the NS workload:
       //      1x2 / 1x4 lanes per face 186 us, 2x2 200 us, 4x4 215 us, 8x2 270 us -- the loop-invariant part of a
       //      face is amortised over more pixels with fewer lanes.)
-#ifndef B200R_SCAN_LANES
-#define B200R_SCAN_LANES 4  // lanes per face (timing experiments: 1, 2)
-#endif
-      constexpr int SL = B200R_SCAN_LANES;
+      constexpr int SL = 4;  // lanes per face (also timed: 1, 2)
       const int dr = tid & (SL - 1);
       for (int fslot = tid / SL; fslot < nc; fslot += FTHREADS / SL) {
         const unsigned rg = sh.rng[fslot];
@@ -854,16 +816,6 @@ __device__ __forceinline__ void fine_tile_body(const FineParams& p, FineStage& s
       // instructions), so that the lanes of a warp evaluate their n-th candidates together whatever words those are
       // in -- looping over the words in lockstep left a third of the lanes active in the evaluation (ncu: 9.8 of 32).
       const float px = sh.col[lc], py = sh.row[lr];
-#ifdef B200R_EXP_OLDWALK  // (timing experiment: the words in lockstep)
-      for (int w = 0; w < nwords; ++w) {
-        unsigned m = sh.u.mask[w][tid];
-        while (m != 0u) {
-          const int j = w * 32 + __ffs((int)m) - 1;
-          m &= m - 1u;
-          consider_face<Q, NB>(sh, j, px, py, blur_radius, persp, clip, q);
-        }
-      }
-#else
       {
         int w = 0;
         unsigned m = sh.u.mask[0][tid];
@@ -875,17 +827,16 @@ __device__ __forceinline__ void fine_tile_body(const FineParams& p, FineStage& s
           consider_face<Q, NB>(sh, j, px, py, blur_radius, persp, clip, q);
         }
       }
-#endif
       continue;  // chunk done
     }
     const float px = sh.col[lc], py = sh.row[lr];
     // (worth its ~80 instructions per face and warp only where a pixel has far more candidates than queue slots: long
     // tile lists -- config 5: 2300 faces per tile, 13.0 -> 9.1 ms; north-star batch with blur 1e-4: none culled, +3 %)
-    const bool cull_depth = (clip || !persp) && (order == ORDER_DEPTH || count >= 512);
+    const bool cull_depth = (clip || !persp) && count >= 512;
     // extent of the warp's footprint (pixel centres are monotonic in the pixel index)
     const float fc0 = sh.col[lc & 8], fc1 = sh.col[(lc & 8) + 7], fr0 = sh.row[lr & 12], fr1 = sh.row[(lr & 12) + 3];
     const float cmin = fminf(fc0, fc1), cmax = fmaxf(fc0, fc1), rmin = fminf(fr0, fr1), rmax = fmaxf(fr0, fr1);
-    const bool warp_active = __any_sync(0xffffffffu, valid);  // (a redo of flagged pixels leaves most warps idle)
+    const bool warp_active = __any_sync(0xffffffffu, valid);  // (false for a warp wholly outside the image)
     for (int sub = 0; sub < nc; sub += ROUND) {
       if (!warp_active) break;
       // ---- pass A: 64-bit mask of the faces of this round whose box contains my pixel
@@ -900,7 +851,6 @@ __device__ __forceinline__ void fine_tile_body(const FineParams& p, FineStage& s
         if (h1) b1 = sh.u.box[sub + 32 + lane];
         // depth culling (see face_depth_lower_bound): once every pixel of the footprint holds K hits
         bool keep0 = h0, keep1 = h1;
-#ifndef B200R_EXP_NOCULL
         if (cull_depth) {
           const float zcut = warp_max(!valid ? -FLT_MAX : (q.full() ? q.max_z() : FLT_MAX));
           if (zcut < FLT_MAX) {
@@ -923,7 +873,6 @@ __device__ __forceinline__ void fine_tile_body(const FineParams& p, FineStage& s
             if (!__any_sync(0xffffffffu, keep0 || keep1)) continue;  // the whole round lies behind the footprint
           }
         }
-#endif
         // (every face of the half-round is either absent / culled or contains the whole footprint)
         const bool all0 =
             __all_sync(0xffffffffu, !keep0 || (cmin >= b0.x && cmax <= b0.y && rmin >= b0.z && rmax <= b0.w));
@@ -963,11 +912,7 @@ __device__ __forceinline__ void fine_tile_body(const FineParams& p, FineStage& s
 // contributes its own view of the flag (the thread that raised it sees it) and nobody reads it after the barrier, which
 // also orders every warp's epilogue reads of the queue payload before the sorted walk reuses shared memory.
 __device__ __forceinline__ bool tile_saw_tie(const FineStage& sh) {
-#ifdef B200R_EXP_NOWATCH
-  return false;
-#else
   return __syncthreads_or(sh.tie) != 0;
-#endif
 }
 
 // Which tile, which faces: grid = (tiles per row, tile rows, images) -- no integer divisions.
@@ -998,24 +943,14 @@ __device__ __forceinline__ TileWork tile_work(const FineParams& p) {
   return t;
 }
 
-// Which walk a tile starts with (see fine_tile_body and DESIGN.md 5).  Without a blur band: arrival order, watched for depth
-// ties.  With one: FRONT TO BACK (ascending nearest-vertex depth) when the depth bound of the warp-level culling exists
-// (clip_barycentric_coords, or no perspective correction) and the list's keys fit the kernel's shared memory -- the queues
-// then fill with near hits first and most of the band's far candidates are culled for whole warps -- again watched for
-// depth ties; the pixels that saw one (only those) are redone in index order before anything is written.  Clipped-face
-// neighbours (order-dependent by themselves) and overflowed tiles: index order.
+// Which walk a tile starts with (see fine_tile_body and DESIGN.md 5): index order for overflowed tiles, for clipped-face
+// neighbours (order-dependent by themselves) and with a blur band; otherwise arrival order, watched for depth ties.
+// (A front-to-back walk of the blur band, with the pixels that saw a tie redone in index order, was measured slower:
+// structured meshes tie so often in the band that too many pixels are redone -- north-star batch with blur 1e-4: fine
+// 917 -> 1306 us, config 2: 139 -> 198 us, config 5: 9.3 -> 14.9 ms.)
 template <bool NB, bool SCAN>
-__device__ __forceinline__ int first_walk_order(const FineParams& p, const TileWork& t) {
-  if (t.overflow || NB) return ORDER_INDEX;
-  if (SCAN) return ORDER_ARRIVAL;
-#ifndef B200R_EXP_DEPTHORDER
-  // (measured, round 2: structured meshes tie so often in the blur band that too many pixels are redone -- north-star
-  // batch with blur 1e-4: fine 917 -> 1306 us, config 2: 139 -> 198 us, config 5: 9.3 -> 14.9 ms; kept as an experiment)
-  return ORDER_INDEX;
-#else
-  const bool bound = p.clip != 0 || p.persp == 0;
-  return (bound && 2 * t.count <= p.smem_ints) ? ORDER_DEPTH : ORDER_INDEX;
-#endif
+__device__ __forceinline__ int first_walk_order(const TileWork& t) {
+  return (t.overflow || NB || !SCAN) ? ORDER_INDEX : ORDER_ARRIVAL;
 }
 
 template <int KMAX, bool NB, bool SCAN>
@@ -1042,24 +977,10 @@ __global__ void __launch_bounds__(FTHREADS, 1024 / FTHREADS) mesh_fine_kernel(co
   float4* pay = rq.pay;
   const int K = p.K;
   // (see fine_tile_body: arrival-order walk first where ties are rare, sorted walk only if one was seen)
-  int order = first_walk_order<NB, SCAN>(p, t);
-  bool active = valid;
-  int scratch_ints = p.smem_ints;
+  int order = first_walk_order<NB, SCAN>(t);
   for (;;) {
   fine_tile_body<RegQueue<KMAX>, NB, SCAN>(p, sh, rq, tile_x, tile_y, n, t.seg_begin, t.count, t.overflow, order,
-                                           active, scratch_ints, lc, lr);
-  if (order == ORDER_DEPTH) {
-    // front-to-back walk done: did any pixel see a depth tie?  Those pixels -- and only those -- walk again in index
-    // order (the queue payload of the others stays where it is: the long-list sort may only use the staging area)
-    if (tile_saw_tie(sh)) {
-      active = valid && sh.tie_lane[tid] != 0;
-      if (active) rq.reset();
-      order = ORDER_INDEX;
-      scratch_ints = (int)(sizeof(FineStage) / sizeof(int));
-      __syncthreads();  // every thread has read its flag before the next walk clears / reuses the staging area
-      continue;
-    }
-  }
+                                           valid, lc, lr);
   bool stored = false;
   int slot[KMAX];
   q.sort(slot);
@@ -1173,22 +1094,10 @@ __global__ void __launch_bounds__(FTHREADS, 768 / FTHREADS) mesh_fine_smemq_kern
 
   SmemQueue<NB> q;
   q.init(smem_raw + sizeof(FineStage), K, tid);
-  int order = first_walk_order<NB, SCAN>(p, t);
-  bool active = valid;
-  int scratch_ints = p.smem_ints;
+  int order = first_walk_order<NB, SCAN>(t);
   for (;;) {
-  fine_tile_body<SmemQueue<NB>, NB, SCAN>(p, sh, q, tile_x, tile_y, n, t.seg_begin, t.count, t.overflow, order, active,
-                                          scratch_ints, lc, lr);
-  if (order == ORDER_DEPTH) {  // (see mesh_fine_kernel)
-    if (tile_saw_tie(sh)) {
-      active = valid && sh.tie_lane[tid] != 0;
-      if (active) q.reset();
-      order = ORDER_INDEX;
-      scratch_ints = (int)(sizeof(FineStage) / sizeof(int));
-      __syncthreads();
-      continue;
-    }
-  }
+  fine_tile_body<SmemQueue<NB>, NB, SCAN>(p, sh, q, tile_x, tile_y, n, t.seg_begin, t.count, t.overflow, order, valid,
+                                          lc, lr);
   q.sort();
   const float px = sh.col[lc], py = sh.row[lr];
   const int64_t o = (((int64_t)n * p.H + yo) * p.W + xo) * K;
@@ -1580,7 +1489,6 @@ __device__ __forceinline__ void warp_scatter(const BackwardParams& p, int face, 
         const int64_t vi = __ldg(fc + j);
         if (vi < 0 || vi >= p.V) continue;  // (out-of-range indices: an error in the reference; ignored like the gather)
         float* o = p.grad_verts + vi * 3;
-#ifndef B200R_EXP_BWD_SCALAR_RED
         if (p.g_vec) {
           const bool odd = (vi & 1) != 0;
           const float s1 = odd ? g[3 * j] : g[3 * j + 2];
@@ -1589,14 +1497,12 @@ __device__ __forceinline__ void warp_scatter(const BackwardParams& p, int face, 
           if (a != 0.0f || b != 0.0f) red_add_v2(o + (odd ? 1 : 0), a, b);
           continue;
         }
-#endif
 #pragma unroll
         for (int c = 0; c < 3; ++c)
           if (g[3 * j + c] != 0.0f) atomicAdd(o + c, g[3 * j + c]);
       }
     } else {
       float* o = p.grad_face_verts + (int64_t)face * 9;
-#ifndef B200R_EXP_BWD_SCALAR_RED
       // (16-byte reductions on the aligned groups inside the 36 bytes -- a four-way switch on face & 3, 3 or 4 reductions per
       // face -- were measured against this: north-star batch with blur 225 vs 215 us, config 5 364 vs 354 us: the divergent
       // switch costs more than the shorter sequences save)
@@ -1608,7 +1514,6 @@ __device__ __forceinline__ void warp_scatter(const BackwardParams& p, int face, 
           red_add_v2(o + 2 * j + odd, odd ? g[2 * j + 1] : g[2 * j], odd ? g[2 * j + 2] : g[2 * j + 1]);
         return;
       }
-#endif
 #pragma unroll
       for (int i = 0; i < 9; ++i) atomicAdd(o + i, g[i]);
     }
@@ -1617,22 +1522,16 @@ __device__ __forceinline__ void warp_scatter(const BackwardParams& p, int face, 
 
 // GV > 0: K is a multiple of GV (8 or 4) and a pixel's face indices are fetched GV at a time with 16-byte loads
 // (a group without faces costs nothing else); GV == 0: any K, scalar loads.
-// PF (GV == 8, 16-byte aligned gradients): valid slots come first in every pixel, so as soon as the indices are known a
-// pixel with a hit fetches the upstream gradients of its first four slots with five 16-byte loads -- one round trip to
-// DRAM for all of them instead of one per slot (the kernel's stall samples are 50 % long_scoreboard: dependent loads).
-#ifndef B200R_BWD_PF_CTAS
-#define B200R_BWD_PF_CTAS 3
-#endif
 // Resident CTAs per SM the register budget is set for.  (Measured on the north-star batch: 4 CTAs, 64 registers: 96.3 us;
 // 5 CTAs, 48 registers, 84 bytes of spills: 135.2 us; 6 CTAs, 40 registers: 163.9 us -- the kernel is bound by load/store
 // instructions through the L1 pipeline, not by the warps in flight: every spill is one more of them.  For the same reason
 // pulling the next wave's indices into L2 with prefetch instructions -- `prefetch.global.L2` of the tile one wave of CTAs
-// ahead -- costs 96.3 -> 100.4 us, and an L1 prefetch of the next slot's face 96.3 -> 100.4 us.)
-#ifndef B200R_BWD_CTAS
-#define B200R_BWD_CTAS 4
-#endif
-template <int GV, bool PF>
-__global__ void __launch_bounds__(TILE_THREADS, PF ? B200R_BWD_PF_CTAS : B200R_BWD_CTAS) mesh_backward_kernel(const BackwardParams p) {
+// ahead -- costs 96.3 -> 100.4 us, and an L1 prefetch of the next slot's face 96.3 -> 100.4 us.  Fetching the upstream
+// gradients of a pixel's first four slots with five 16-byte loads as soon as the indices are known -- one DRAM round trip
+// instead of one per slot -- needs 80 registers, three CTAs: 96 -> 113 us.)
+constexpr int BWD_CTAS = 4;
+template <int GV>
+__global__ void __launch_bounds__(TILE_THREADS, BWD_CTAS) mesh_backward_kernel(const BackwardParams p) {
   const int lane = threadIdx.x & 31;
   const int tile_x = blockIdx.x, tile_y = blockIdx.y, n = p.n0 + blockIdx.z;  // grid = (TX, TY, images)
   int xo, yo;
@@ -1644,7 +1543,6 @@ __global__ void __launch_bounds__(TILE_THREADS, PF ? B200R_BWD_PF_CTAS : B200R_B
   const int64_t o = in_image ? (((int64_t)n * p.H + yo) * p.W + xo) * K : 0;
   const bool persp = p.persp != 0, clip = p.clip != 0;
   constexpr int G = GV > 0 ? GV : 1;
-  static_assert(!PF || GV == 8, "the prefetching variant is the K % 8 == 0 kernel");
 
   for (int k0 = 0; k0 < K; k0 += G) {
     int fk[G];
@@ -1659,51 +1557,21 @@ __global__ void __launch_bounds__(TILE_THREADS, PF ? B200R_BWD_PF_CTAS : B200R_B
     } else {
       fk[0] = in_image ? (int)p.pix_to_face[o + k0] : -1;
     }
-    float pz[PF ? 4 : 1], pd[PF ? 4 : 1], pb[PF ? 12 : 1];  // upstream gradients of slots k0 .. k0+3
-    if (PF) {
-      float4 vz = make_float4(0.f, 0.f, 0.f, 0.f), vd = vz, b0 = vz, b1 = vz, b2 = vz;
-      if (fk[0] >= 0) {
-        vz = __ldg(reinterpret_cast<const float4*>(p.grad_zbuf + o + k0));
-        vd = __ldg(reinterpret_cast<const float4*>(p.grad_dists + o + k0));
-        const float4* gb = reinterpret_cast<const float4*>(p.grad_bary + (o + k0) * 3);
-        b0 = __ldg(gb + 0);
-        b1 = __ldg(gb + 1);
-        b2 = __ldg(gb + 2);
-      }
-      pz[0] = vz.x; pz[1] = vz.y; pz[2] = vz.z; pz[3] = vz.w;
-      pd[0] = vd.x; pd[1] = vd.y; pd[2] = vd.z; pd[3] = vd.w;
-      pb[0] = b0.x; pb[1] = b0.y; pb[2] = b0.z; pb[3] = b0.w;
-      pb[4] = b1.x; pb[5] = b1.y; pb[6] = b1.z; pb[7] = b1.w;
-      pb[8] = b2.x; pb[9] = b2.y; pb[10] = b2.z; pb[11] = b2.w;
-    }
 #pragma unroll 1
     for (int j = 0; j < G; ++j) {
       const int face = fk[0];
 #pragma unroll
       for (int u = 0; u + 1 < G; ++u) fk[u] = fk[u + 1];  // rotate: one copy of the gradient code
-      float gz = 0.f, gd = 0.f, gb0 = 0.f, gb1 = 0.f, gb2 = 0.f;
-      if (PF) {  // (rotated like the indices)
-        gz = pz[0]; gd = pd[0]; gb0 = pb[0]; gb1 = pb[1]; gb2 = pb[2];
-#pragma unroll
-        for (int u = 0; u < 3; ++u) {
-          pz[u] = pz[u + 1];
-          pd[u] = pd[u + 1];
-        }
-#pragma unroll
-        for (int u = 0; u < 9; ++u) pb[u] = pb[u + 3];
-      }
       if (!__any_sync(0xffffffffu, face >= 0)) continue;  // padded slots (:472-474)
       float g[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
       if (face >= 0) {
         const int64_t i = o + k0 + j;
-        if (!PF || j >= 4) {
-          gz = __ldg(p.grad_zbuf + i);
-          gd = __ldg(p.grad_dists + i);
-          // (8 + 4 byte loads of the three barycentric gradients instead of three scalar ones: 94.2 -> 98.4 us, more spills)
-          gb0 = __ldg(p.grad_bary + i * 3);
-          gb1 = __ldg(p.grad_bary + i * 3 + 1);
-          gb2 = __ldg(p.grad_bary + i * 3 + 2);
-        }
+        const float gz = __ldg(p.grad_zbuf + i);
+        const float gd = __ldg(p.grad_dists + i);
+        // (8 + 4 byte loads of the three barycentric gradients instead of three scalar ones: 94.2 -> 98.4 us, more spills)
+        const float gb0 = __ldg(p.grad_bary + i * 3);
+        const float gb1 = __ldg(p.grad_bary + i * 3 + 1);
+        const float gb2 = __ldg(p.grad_bary + i * 3 + 2);
         backward_one(p, px, py, face, gz, gd, gb0, gb1, gb2, persp, clip, g);
       }
       warp_scatter(p, face, g, lane);
@@ -1764,39 +1632,27 @@ static int forward_impl(const float* face_verts, const float* verts, int64_t V, 
 
   const bool prof = profiling_enabled();
   if (prof) phase_timer().record(0, stream);
-#ifndef B200R_EXP_MEMSET_NODE
   zero_ints_kernel<<<(unsigned)((ntiles + 1023) / 1024), 256, 0, stream>>>(ws.tile_count, ntiles);
   B200R_LAUNCHED("zero_ints_kernel");
-#else
-  B200R_CUDA_OK(cudaMemsetAsync(ws.tile_count, 0, sizeof(int) * (size_t)ntiles, stream));
-#endif
   if (F > 0) {
-    const unsigned sgrid = (unsigned)((F + SETUP_FACES - 1) / SETUP_FACES);
-#ifndef B200R_EXP_MEMSET_NODE
-#define B200R_SETUP_LAUNCH(KERNEL, ...) B200R_CUDA_OK(launch_chained(KERNEL, dim3(sgrid), dim3(SETUP_FACES), 0, stream, __VA_ARGS__))
-#else
-#define B200R_SETUP_LAUNCH(KERNEL, ...) KERNEL<<<sgrid, SETUP_FACES, 0, stream>>>(__VA_ARGS__)
-#endif
+    const dim3 sgrid((unsigned)((F + SETUP_FACES - 1) / SETUP_FACES));
     if (faces != nullptr) {
-      B200R_SETUP_LAUNCH(mesh_setup_count_kernel<true>, (const float*)nullptr, verts, V, faces, face_verts_out, neighbor, F,
-                         first, num, N, H, W, TY, TX, rx, ry, sqrt_blur, cull_backfaces, ws.rect, ws.tile_count, rec);
+      B200R_CUDA_OK(launch_chained(mesh_setup_count_kernel<true>, sgrid, dim3(SETUP_FACES), 0, stream,
+                                   (const float*)nullptr, verts, V, faces, face_verts_out, neighbor, F, first, num, N, H,
+                                   W, TY, TX, rx, ry, sqrt_blur, cull_backfaces, ws.rect, ws.tile_count, rec));
       face_verts = face_verts_out;
     } else {
-      B200R_SETUP_LAUNCH(mesh_setup_count_kernel<false>, face_verts, (const float*)nullptr, (int64_t)0,
-                         (const int64_t*)nullptr, (float*)nullptr, neighbor, F, first, num, N, H, W, TY, TX, rx, ry,
-                         sqrt_blur, cull_backfaces, ws.rect, ws.tile_count, rec);
+      B200R_CUDA_OK(launch_chained(mesh_setup_count_kernel<false>, sgrid, dim3(SETUP_FACES), 0, stream, face_verts,
+                                   (const float*)nullptr, (int64_t)0, (const int64_t*)nullptr, (float*)nullptr,
+                                   neighbor, F, first, num, N, H, W, TY, TX, rx, ry, sqrt_blur, cull_backfaces, ws.rect,
+                                   ws.tile_count, rec));
     }
-#undef B200R_SETUP_LAUNCH
     B200R_LAUNCHED("mesh_setup_count_kernel");
   }
   // Schedule of the fine pass (see tile_scan_kernel): worth the extra pass of the scan kernel and one more dependent load
   // per CTA where tiles run long -- with a blur band (north-star batch + blur 1e-4: fine 918 -> 749 us, config 2: 137 ->
   // 109 us); without one the north-star batch loses 6 us.  The packed class counters hold 2^21 tiles.
-#ifdef B200R_EXP_NOTILEORDER
-  int* const tile_order = nullptr;
-#else
   int* const tile_order = (blur_radius > 0.0f && ntiles < (1ll << ORDER_BITS)) ? ws.tile_order : nullptr;
-#endif
   B200R_CUDA_OK(launch_chained(tile_scan_kernel, dim3(1), dim3(1024), 0, stream, ws.tile_count, ws.tile_offset,
                                (int)ntiles, tile_order));
   B200R_LAUNCHED("tile_scan_kernel");
@@ -1952,21 +1808,12 @@ static int backward_impl(const float* face_verts, int64_t F, const int64_t* pix_
   if (prof) phase_timer().record(3, stream);
   for (p.n0 = 0; p.n0 < N; p.n0 += 65535) {  // grid.z is limited to 65535 images per launch
     const dim3 bgrid((unsigned)TX, (unsigned)TY, (unsigned)min(N - p.n0, 65535));
-    const bool aligned = ((reinterpret_cast<uintptr_t>(grad_zbuf) | reinterpret_cast<uintptr_t>(grad_bary) |
-                           reinterpret_cast<uintptr_t>(grad_dists)) & 15u) == 0;
-#ifdef B200R_EXP_BWDPF  // (measured, round 2: 96 -> 113 us at three CTAs per SM: the occupancy it costs outweighs the
-    const bool prefetch = aligned;  // round trips it saves; kept as an experiment)
-#else
-    const bool prefetch = false && aligned;
-#endif
-    if ((K & 7) == 0 && prefetch)
-      mesh_backward_kernel<8, true><<<bgrid, TILE_THREADS, 0, stream>>>(p);
-    else if ((K & 7) == 0)
-      mesh_backward_kernel<8, false><<<bgrid, TILE_THREADS, 0, stream>>>(p);
+    if ((K & 7) == 0)
+      mesh_backward_kernel<8><<<bgrid, TILE_THREADS, 0, stream>>>(p);
     else if ((K & 3) == 0)
-      mesh_backward_kernel<4, false><<<bgrid, TILE_THREADS, 0, stream>>>(p);
+      mesh_backward_kernel<4><<<bgrid, TILE_THREADS, 0, stream>>>(p);
     else
-      mesh_backward_kernel<0, false><<<bgrid, TILE_THREADS, 0, stream>>>(p);
+      mesh_backward_kernel<0><<<bgrid, TILE_THREADS, 0, stream>>>(p);
   }
   B200R_LAUNCHED("mesh_backward_kernel");
   if (prof) {

@@ -55,9 +55,7 @@ __global__ void __launch_bounds__(SETUP_POINTS)
     rect[pi] = make_uint4(rc.x, rc.y, (uint32_t)max(n, 0), 0u);
     prec[pi] = make_float4(x, y, z, r);
   }
-#ifndef B200R_EXP_MEMSET_NODE
   pdl_wait();  // the counters are zeroed by the kernel this one is chained to (see zero_ints_kernel)
-#endif
   warp_count_rect<false>(rc, n, TY, TX, tile_count, tid & 31);
 }
 
@@ -75,7 +73,6 @@ __global__ void __launch_bounds__(256)
   // all of the thread's points first (one round trip to DRAM for the chunk instead of one per point: the loads were 31 % of
   // the kernel's stall samples when each iteration waited for its own)
   float xs[BIN_CHUNK / 256], ys[BIN_CHUNK / 256], zs[BIN_CHUNK / 256], rs[BIN_CHUNK / 256];
-#ifndef B200R_EXP_PSETUP_NOHOIST
 #pragma unroll
   for (int i = 0; i < BIN_CHUNK / 256; ++i) {
     const int64_t pi = p0 + i * 256 + tid;
@@ -87,25 +84,16 @@ __global__ void __launch_bounds__(256)
       rs[i] = __ldg(radius + pi);
     }
   }
-#endif
   for (int t = tid; t < T; t += 256) hist[t] = 0;
   const int n0 = find_owner(first, num, N, p0);  // the chunk's image (uniform); -1: the chunk starts in a gap
   const int64_t lo0 = n0 >= 0 ? __ldg(first + n0) : 0, hi0 = n0 >= 0 ? lo0 + __ldg(num + n0) : 0;
   __syncthreads();
-#ifndef B200R_EXP_MEMSET_NODE
   pdl_wait();  // the counters are zeroed by the kernel this one is chained to (see zero_ints_kernel)
-#endif
 #pragma unroll
   for (int i = 0; i < BIN_CHUNK / 256; ++i) {
     const int64_t pi = p0 + i * 256 + tid;
     if (pi >= P) continue;
-#ifndef B200R_EXP_PSETUP_NOHOIST
     const float x = xs[i], y = ys[i], z = zs[i], r = rs[i];
-#else
-    (void)xs; (void)ys; (void)zs; (void)rs;
-    const float x = __ldg(points + pi * 3 + 0), y = __ldg(points + pi * 3 + 1), z = __ldg(points + pi * 3 + 2);
-    const float r = __ldg(radius + pi);
-#endif
     const int n = (pi >= lo0 && pi < hi0) ? n0 : find_owner(first, num, N, pi);
     uint2 rc = make_uint2(RECT_EMPTY_X, 0u);
     if (n >= 0 && !(z < 0.0f)) rc = bbox_to_tile_rect(fsub(x, r), fadd(x, r), fsub(y, r), fadd(y, r), H, W, rx, ry);
@@ -365,11 +353,7 @@ __global__ void __launch_bounds__(TILE_THREADS) points_fine_smem_kernel(const Po
   int size, max_idx;
   float max_z;
   const int seg_begin0 = p.tile_offset[tile], seg_end0 = p.tile_offset[tile + 1];
-#ifdef B200R_EXP_NOBYDEPTH  // (timing experiment: arrival-order walk with the literal queue first)
-  const bool by_depth_ok = false;
-#else
   const bool by_depth_ok = !((int64_t)seg_end0 > p.capacity || seg_end0 == INT_MAX) && seg_end0 - seg_begin0 <= PCHUNK;
-#endif
   for (int attempt = by_depth_ok ? 0 : 1;; attempt = 2) {  // 0: depth order, 1: arrival order, 2: index order (exact)
     const bool sort_list = attempt == 2;
     size = 0;
@@ -636,7 +620,6 @@ __global__ void __launch_bounds__(TILE_THREADS)
     }
     if (pi >= 0 && lane == __ffs((int)grp) - 1) {
       float* o = grad_points + (int64_t)pi * 3;
-#ifndef B200R_EXP_BWD_SCALAR_RED
       if (g_vec) {
         // (a point's 12 bytes start at a multiple of 4 whose parity is that of the index: one 8-byte vector reduction and
         // one scalar one instead of three -- fewer instructions through the L1 / MIO pipeline, the same sums)
@@ -644,9 +627,7 @@ __global__ void __launch_bounds__(TILE_THREADS)
         atomicAdd(o + (odd ? 0 : 2), odd ? gx : gz);
         asm volatile("red.global.add.v2.f32 [%0], {%1, %2};" ::"l"(o + (odd ? 1 : 0)), "f"(odd ? gy : gx), "f"(odd ? gz : gy)
                      : "memory");
-      } else
-#endif
-      {
+      } else {
         atomicAdd(o + 0, gx);
         atomicAdd(o + 1, gy);
         atomicAdd(o + 2, gz);
@@ -692,12 +673,8 @@ extern "C" int b200r_rasterize_points_forward(const float* points, int64_t P, co
 
   const bool prof = profiling_enabled();
   if (prof) phase_timer().record(0, stream);
-#ifndef B200R_EXP_MEMSET_NODE
   zero_ints_kernel<<<(unsigned)((ntiles + 1023) / 1024), 256, 0, stream>>>(ws.tile_count, ntiles);
   B200R_LAUNCHED("zero_ints_kernel");
-#else
-  B200R_CUDA_OK(cudaMemsetAsync(ws.tile_count, 0, sizeof(int) * (size_t)ntiles, stream));
-#endif
   // (a private histogram over one image's tiles per CTA, if it fits; see binning.cuh)
   const bool private_hist = (int64_t)TY * TX <= BIN_MAX_TILES;
   const size_t hist_bytes = sizeof(int) * (size_t)TY * TX;

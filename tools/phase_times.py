@@ -1,6 +1,8 @@
 """Step time and binning / fine / backward phase times (CUDA events inside the library) of workloads of bench.py.
 
-    python tools/phase_times.py [--lib path/to/variant.so] [--pdl 0|1|both] ns c2 ns_blur c5 c3
+    python tools/phase_times.py [--pdl 0|1|both] ns c2 ns_blur c5 c3
+
+(B200R_LIB=<path> times another build of the library, see pytorch3d_b200/_lib.py.)
 """
 import ctypes
 import os
@@ -16,10 +18,7 @@ from pytorch3d_b200 import _C, _lib, synthetic  # noqa: E402
 args = sys.argv[1:]
 pdl_modes = [1]
 while args and args[0].startswith("--"):
-    if args[0] == "--lib":  # development: time another build of the library (through the ctypes binding: the
-        _lib.LIB_PATH = os.path.abspath(args[1])  # torch extension is linked against the in-tree library)
-        _C.USE_EXT = False
-    elif args[0] == "--pdl":
+    if args[0] == "--pdl":
         pdl_modes = [0, 1] if args[1] == "both" else [int(args[1])]
     args = args[2:]
 dev = torch.device("cuda:0")
